@@ -59,7 +59,15 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--hf-gpu-batches", type=int, default=2, help="timed 256-prompt batches of the HF-eager-on-GPU incumbent (0 = skip)")
     ap.add_argument("--parity-rows", type=int, default=16, help="rows of the last timed batch checked against HF on this GPU (0 = skip)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the tokens generate() returned in the last timed step (rank 0) as "
+                         "DIR/generated_tokens.npy (float32), so that two builds can be compared on identical seeded inputs")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return a
 
 
 def dist_env():
@@ -142,24 +150,19 @@ class ClockSampler:
 
 # --------------------------------------------------------------------------- CPU path (reference arm / baseline)
 def _cpu_predictor(a):
-    """HF eager fp32 model behind the predictor plug-in: the reference's OWN predictor.py when its checkout is
-    present (kind "reference"), this package's mirror of it otherwise (kind "port"; the arithmetic is the genuine
-    dependency either way)."""
+    """HF eager fp32 model behind this package's mirror of the reference's predictor plug-in (kind "port"; the
+    arithmetic is the genuine dependency, and tests/test_reference_predictor_cpu.py pins the mirror to the
+    reference's own class output for output)."""
     import torch
     from transformers import T5Tokenizer
 
-    from anyscale_workshop_nyc_2023_b200 import refsource
+    from anyscale_workshop_nyc_2023_b200.predictor import HuggingFaceModelPredictor
     from anyscale_workshop_nyc_2023_b200.workload import checkpoint_dir
     from oracle.hf_anchor import load_hf_model
 
     ckpt = checkpoint_dir(a.model, seed=0)
     model = load_hf_model(ckpt, dtype=torch.float32, device="cpu")
     tok = T5Tokenizer.from_pretrained(str(ckpt))
-    ref = refsource.load_reference_predictor_module()
-    if ref is not None:
-        return ref.HuggingFaceModelPredictor(model, tokenizer=tok), "reference"
-    from anyscale_workshop_nyc_2023_b200.predictor import HuggingFaceModelPredictor
-
     return HuggingFaceModelPredictor(model, tokenizer=tok), "port"
 
 
@@ -206,7 +209,7 @@ def run_cpu_path(a, steps: int, warmup: int, sample: int):
     toks = steps * sample * a.new
     return {"value": toks / total, "unit": UNIT, "cores": threads, "kind": kind,
             "sample": f"{steps} step(s) x one batch of {sample} prompts of the same {a.seq}->{a.new} workload, HF transformers eager "
-                      f"fp32 generate via {'the reference predictor.py' if kind == 'reference' else 'the predictor plug-in mirror'}, "
+                      "fp32 generate via the predictor plug-in mirror, "
                       f"torch threads={threads} (3-point sweep {dict((k, round(v, 2)) for k, v in sweep.items())} s per probe; "
                       f"{cores} usable cores)",
             "prompts_per_s": steps * sample / total, "ms_per_step": 1e3 * total / steps,
@@ -217,7 +220,7 @@ def main_reference(a):
     rank, world, _ = dist_env()
     if rank != 0:
         return 0
-    steps = max(a.steps, 1)
+    steps = a.steps
     warm = min(a.warmup, 1)  # CPU steps are seconds long; at most one warm-up pass
     # bounded: one 64-prompt batch per step for short runs, smaller batches when the driver asks for many steps
     sample = a.cpu_sample if steps <= 3 else max(8, min(a.cpu_sample, 16))
@@ -316,6 +319,23 @@ def hf_gpu_legs(a, ckpt, spec, last_batch, last_out, dtype, model=None):
 
 
 # --------------------------------------------------------------------------- B200 arm
+DUMP_LIMIT_BYTES = 60 << 20  # keeps a dump under 64 MB, .npy headers included
+
+
+def dump_tokens(out_dir: Path, tokens):
+    """Token ids (< 2**24, exact in float32) as out_dir/generated_tokens.npy; above DUMP_LIMIT_BYTES a fixed seeded
+    sample of rows, in row order, with their indices in out_dir/generated_tokens_rows.npy."""
+    import numpy as np
+
+    out_dir.mkdir(parents=True, exist_ok=True)
+    rows = DUMP_LIMIT_BYTES // (4 * tokens.shape[1] + 8)
+    if tokens.shape[0] > rows:
+        keep = np.sort(np.random.default_rng(0).choice(tokens.shape[0], rows, replace=False))
+        tokens = tokens[keep]
+        np.save(out_dir / "generated_tokens_rows.npy", keep.astype(np.float64))
+    np.save(out_dir / "generated_tokens.npy", tokens.astype(np.float32))
+
+
 def main_b200(a):
     import numpy as np
     import torch
@@ -400,6 +420,8 @@ def main_b200(a):
     elapsed_ms = e0.elapsed_time(e1)
     clocks = sampler.stop()
     last_out = out.cpu().numpy()  # the last TIMED batch's tokens: checked against HF below, outside the timed region
+    if a.dump_outputs and rank == 0:
+        dump_tokens(Path(a.dump_outputs), last_out)
 
     if rank == 0:
         log(f"device-resident: {elapsed_ms / K:.1f} ms/step")

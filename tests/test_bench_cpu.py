@@ -42,3 +42,28 @@ def test_product_arm_fails_loudly_without_a_gpu():
     assert proc.returncode != 0
     assert "no CPU fallback" in (proc.stderr + proc.stdout) or "CUDA" in (proc.stderr + proc.stdout)
     assert not any(ln.lstrip().startswith("{") for ln in proc.stdout.splitlines())  # no number is reported
+
+
+def test_dump_outputs_writes_the_tokens_and_stays_under_its_limit(tmp_path, monkeypatch):
+    import numpy as np
+
+    import bench
+
+    tokens = np.arange(6 * 9).reshape(6, 9)
+    bench.dump_tokens(tmp_path / "all", tokens)
+    assert sorted(p.name for p in (tmp_path / "all").iterdir()) == ["generated_tokens.npy"]
+    got = np.load(tmp_path / "all" / "generated_tokens.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, tokens)
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 3 * (4 * 9 + 8))
+    for d in ("s1", "s2"):
+        bench.dump_tokens(tmp_path / d, tokens)
+    rows = np.load(tmp_path / "s1" / "generated_tokens_rows.npy").astype(int)
+    assert len(rows) == 3 and (np.diff(rows) > 0).all()
+    assert np.array_equal(np.load(tmp_path / "s1" / "generated_tokens.npy"), tokens[rows])
+    assert np.array_equal(rows, np.load(tmp_path / "s2" / "generated_tokens_rows.npy"))  # the same sample every run
+
+
+def test_bench_rejects_zero_steps_and_dumps_on_the_reference_arm(tmp_path):
+    for args in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        proc = run_bench(*args, timeout=120)
+        assert proc.returncode == 2 and "error:" in proc.stderr and not proc.stdout.strip()

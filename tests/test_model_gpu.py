@@ -343,7 +343,7 @@ def test_batch_predictor_api_single_gpu(models):
     assert out["generated_output"].tolist() == want
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 def test_batch_predictor_pool_two_gpus():
     """One scoring process per GPU, blocks dealt round-robin, results back in input order."""
     from anyscale_workshop_nyc_2023_b200 import rayshim

@@ -50,7 +50,9 @@ def test_visible_devices_are_passed_through_as_strings(monkeypatch):
 
 
 @pytest.mark.timeout(300)
-def test_pool_order_persistence_and_worker_side_cpu_stage():
+def test_pool_order_persistence_and_worker_side_cpu_stage(monkeypatch):
+    # two devices for the two workers whatever this host has (the stand-in predictor never touches them)
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "0,1")
     with GpuWorkerPool(2, Ckpt(), EchoPredictor, {}, True) as pool:
         outs = pool.map_ordered(_blocks(7), None, None, {"suffix": "x"})
         assert [o["generated_output"].tolist() for o in outs] == [[f"b{i}r{j}:x" for j in range(3)] for i in range(7)]
